@@ -2,7 +2,7 @@
 """bench.py — DDPM 256x256 denoising steps/sec @ 1.2 % edit (BASELINE.json metric), B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-cuda] [--ratio 0.012]
-                    [--path fused|modules] [--no-flush]
+                    [--path fused|modules] [--no-flush] [--dump-outputs DIR]
 
 One "step" = one SPARSE forward of the DDPM U-Net on the edited latent with pre-filled caches —
 what the reference's Runner.profile times (reference diffusion/runner.py:214-245).  Workload =
@@ -94,9 +94,36 @@ def parse():
     ap.add_argument("--ksplit", type=int, default=0, help="engine: force the split-K factor (0 = auto)")
     ap.add_argument("--no-graph", action="store_true", help="launch the step eagerly instead of replaying a CUDA graph")
     ap.add_argument("--ncu", action="store_true",
-                    help="profiling aid: after warm-up run --steps eager steps between cudaProfilerStart/Stop and exit "
+                    help="profiling aid: after warm-up run one eager step between cudaProfilerStart/Stop and exit "
                          "(use with `ncu --profile-from-start off`); prints no bench line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned to its caller as DIR/<name>.npy (float32, "
+                         "at most 64 MB in all: a larger output is cut to a fixed, seeded sample); the inputs are seeded, so two "
+                         "builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes this repository's outputs (--impl ours)")
+    if args.dump_outputs and args.ncu:
+        ap.error("--ncu runs no timed steps: there is nothing for --dump-outputs to write")
+    return args
+
+
+def dump_outputs(directory, arrays, limit=64 * 10 ** 6):
+    """Write each array as directory/<name>.npy in float32.  When the arrays together exceed `limit` bytes, each one is
+    replaced by the same fixed, seeded sample of its flattened elements (in index order), in proportion to its size."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > limit:
+            keep = a.size * (limit - 4096 * len(arrays)) // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
+    log("outputs of the last timed step written to %s: %s" % (directory, ", ".join(sorted(arrays))))
 
 
 # ------------------------------------------------------------------------------------------
@@ -263,9 +290,9 @@ def run_reference(args):
     if args._cpu_child:
         print(json.dumps(cpu_reference_legacy(args.ratio, max(1, args.steps), max(1, args.warmup), args.threads)), flush=True)
         return
-    steps = max(1, min(args.steps, 40))          # each step is a bounded sample: the whole arm ends within a few minutes
     warm = max(1, min(args.warmup, 5))
-    r = cpu_reference_subprocess(args.ratio, steps, warm, threads=args.threads)
+    # the time limit grows with --steps (a few seconds per step is ample for the host-core flow), so every step asked for is timed
+    r = cpu_reference_subprocess(args.ratio, args.steps, warm, timeout=170 + 5 * args.steps, threads=args.threads)
     line = {
         "impl": "reference", "metric": "DDPM 256x256 denoising steps/sec @1.2% edit", "value": r["value"], "unit": "steps/s",
         "n_gpus": args.gpus, "steps": r["timed_steps"], "warmup": r.get("warmup", warm), "ms_per_step": r["ms_per_step"],
@@ -496,6 +523,9 @@ def run_ours(args):
     ms = region(args.steps, False)
     ms_e2e = region(args.steps, True)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        # out_host holds eps of the last end-to-end step: what a caller of the public call receives
+        dump_outputs(args.dump_outputs, {"eps" if world == 1 else "eps_rank%d" % rank: out_host.numpy()}, limit=64 * 10 ** 6 // world)
 
     value = world * n_edits * args.steps / (ms / 1e3)            # denoising steps of ONE edit per second, summed over edits and GPUs
     e2e_value = world * n_edits * args.steps / (ms_e2e / 1e3)
@@ -588,7 +618,7 @@ def run_consumer(args):
     ref = None
     if loader.available(cuda=True):
         dump = os.path.join(tempfile.mkdtemp(prefix="sige_ref_"), "ref.npz")
-        r = _reference_child("cuda", args.ratio, max(1, min(args.steps, 20)), 3, 0, 900, extra=["--workload", args.workload])      # stock settings (TF32 convs): the timing
+        r = _reference_child("cuda", args.ratio, args.steps, 3, 0, 900 + 5 * args.steps, extra=["--workload", args.workload])      # stock settings (TF32 convs): the timing
         _reference_child("cuda", args.ratio, 1, 1, 0, 900, extra=["--workload", args.workload, "--no-tf32", "--dump", dump])         # exact fp32: the parity target
         ref = (r, np.load(dump))
         log("reference CUDA path: %.2f ms/step" % r["ms_per_step"])
@@ -611,7 +641,7 @@ def run_consumer(args):
         return sum(a.elapsed_time(b) for a, b in evs) / k, out
 
     timed(3)
-    ms_mod, out_mod = timed(max(3, min(args.steps, 20)))
+    ms_mod, out_mod = timed(args.steps)
     net.set_fused(True, dtype=dtype)
     t0 = time.time()
     with torch.no_grad():
@@ -619,7 +649,9 @@ def run_consumer(args):
     compile_s = time.time() - t0
     step = net.fused_step
     timed(3)
-    ms_fused, out_fused = timed(max(5, min(args.steps, 50)))
+    ms_fused, out_fused = timed(args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"out": out_fused.float().cpu().numpy()})
 
     def rel(a, b):
         return float(np.abs(a - b).max() / np.abs(b).max())
@@ -636,6 +668,7 @@ def run_consumer(args):
             "gaugan": "GauGAN SPADE generator (ngf 64, 'more' up-sampling), 512x1024, 2.98 % label edit"}[args.workload]
     line = {
         "metric": "%s sparse steps/sec" % args.workload, "value": 1e3 / ms_fused, "unit": "steps/s", "n_gpus": 1, "ms_per_step": ms_fused,
+        "steps": args.steps, "warmup": 3,
         "higher_is_better": True, "dtype": "f16" if dtype == torch.float16 else "bf16", "data": "synthetic (random-init weights)",
         "config": {"workload": name, "model_file": "the reference's unmodified model file (baseline/_ref) on this repo's sige.nn",
                    "path": ("model(...) as a fused step: %d fused conv launches + %d sige_sparse_attention + %d sige_spade_modulate launches + %d recorded torch calls in one CUDA graph"

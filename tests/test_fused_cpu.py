@@ -203,7 +203,7 @@ def test_batch_of_independent_edits_equals_one_edit_at_a_time():
     from sim_executor import SimExecutor
 
     cfg = DDPMConfig.small()
-    model, _, t = _prepared("reference", cfg, 0.05)
+    model, _, t = _prepared("intree", cfg, 0.05)
     edits = []
     for e, (ratio, shift) in enumerate([(0.05, (0, 0)), (0.02, (-14, 9)), (0.09, (11, -13))]):
         x0, x1, mask, _ = synthetic_inputs(cfg, ratio, seed=0, edit_seed=e)
@@ -239,7 +239,7 @@ def test_new_masks_are_installed_without_recompiling():
     from sim_executor import SimExecutor
 
     cfg = DDPMConfig.small()
-    model, x_a, t = _prepared("reference", cfg, 0.05)
+    model, x_a, t = _prepared("intree", cfg, 0.05)
     x0, _, _, _ = synthetic_inputs(cfg, 0.05, seed=0)
     with torch.no_grad():
         step = FusedStep(model, x_a, t, executor=SimExecutor())

@@ -1,16 +1,14 @@
-"""The fused step (sige_b200.fused) on the GPU: the reference's UNMODIFIED model file and the in-tree workload,
-through the public call ``model(x, t)``, against the reference's golden outputs (tests/golden/*.npz)."""
-import os
-import sys
+"""The fused step (sige_b200.fused) on the GPU: the DDPM U-Net of the in-tree workload (the reference's architecture, its
+parameter names and weights), through the public call ``model(x, t)``, against the reference's golden outputs
+(tests/golden/*.npz)."""
 import warnings
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import REPO, golden
+from conftest import golden
 
-sys.path.insert(0, os.path.join(REPO, "baseline"))
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 
@@ -26,28 +24,21 @@ def _exact_fp32_dense_pass():
     torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = saved
 
 
-def _model(kind, cfg):
-    import loader
+def _model(cfg):
     from sige_b200.workloads.ddpm import SIGEDDPMUNet, init_deterministic
 
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
-        if kind == "reference":
-            assert loader.available(), "baseline/_ref did not travel (python baseline/build_ref.py builds it where /root/reference exists)"
-            model = loader.reference_ddpm_on_this_repo(cfg)
-        else:
-            model = SIGEDDPMUNet(cfg)
-        return init_deterministic(model, seed=0).eval()
+        return init_deterministic(SIGEDDPMUNet(cfg), seed=0).eval()
 
 
-def _prepared(kind, cfg, ratio, dtype, channels_last=True):
+def _prepared(cfg, ratio, dtype, channels_last=True):
     """dtype fp32: the reference's own flow — fp32 model, fp32 dense pass — with the sparse steps opted into fp16 tensor-core
-    arithmetic (set_fused(dtype=...)); dtype fp16: a half model end to end (the in-tree workload supports it; the
-    reference's model file computes its time embedding in fp32 and cannot run its dense pass in half)."""
+    arithmetic (set_fused(dtype=...)); dtype fp16: a half model end to end."""
     from sige.utils import downsample_mask
     from sige_b200.workloads.ddpm import synthetic_inputs
 
-    model = _model(kind, cfg).to(DEV).to(dtype)
+    model = _model(cfg).to(DEV).to(dtype)
     if channels_last:
         model = model.to(memory_format=torch.channels_last)
     x0, x1, mask, t = synthetic_inputs(cfg, ratio, seed=0)
@@ -76,15 +67,14 @@ TOL_MAX, TOL_RMS, TOL_REL = 5e-3, 6e-4, 5e-2
 
 
 @pytest.mark.parametrize("channels_last", [False, True])
-def test_reference_model_file_unmodified_runs_fused(channels_last):
-    """north star: the reference's own diffusion/models/ddpm_arch/sige_fused_unet.py, unmodified, on this repo's sige.nn:
-    full -> set_masks -> sparse through model(x, t); the sparse call is ONE fused launch per wrapped layer."""
+def test_ddpm256_model_runs_fused(channels_last):
+    """north star: the DDPM-256 U-Net on this repo's sige.nn, full -> set_masks -> sparse through model(x, t); the sparse
+    call is ONE fused launch per wrapped layer."""
     from sige_b200.parallel import cache_tensors
     from sige_b200.workloads.ddpm import DDPMConfig
 
     G = golden("ddpm256_golden.npz")
-    model, x1, t = _prepared("reference", DDPMConfig(), float(G["ratio"][0]), torch.float32, channels_last)
-    assert type(model).__module__ == "models.ddpm_arch.sige_fused_unet"
+    model, x1, t = _prepared(DDPMConfig(), float(G["ratio"][0]), torch.float32, channels_last)
     pristine = [(n, v.clone()) for n, v in cache_tensors(model)]
     with torch.no_grad():
         out1 = model(x1, t)
@@ -105,7 +95,7 @@ def test_reference_model_file_unmodified_runs_fused(channels_last):
     for (n, a), (_, b) in zip(pristine, cache_tensors(model)):
         assert torch.equal(a, b), "the fused step must not touch the module caches (%s)" % n
     e_max, e_rms, e_rel = _errs(out1.float().cpu().numpy(), G["sparse_out"])
-    print("reference model fused (channels_last=%s): max %.3g rms %.3g rel %.3g, %d launches/step" % (channels_last, e_max, e_rms, e_rel, step.launches_per_step))
+    print("DDPM-256 model fused (channels_last=%s): max %.3g rms %.3g rel %.3g, %d launches/step" % (channels_last, e_max, e_rms, e_rel, step.launches_per_step))
     assert e_max <= TOL_MAX and e_rms <= TOL_RMS and e_rel <= TOL_REL
     # the eager fp32 operator modules reproduce the reference to fp32 accuracy; the fp16 fused step stays within the fp16 tolerance of them
     model.set_fused(False)
@@ -137,7 +127,7 @@ def test_fused_step_options_vs_modules_and_reference(tag, opts):
 
     G = golden(tag + "_golden.npz")
     cfg = DDPMConfig.small() if tag == "ddpm_small" else DDPMConfig()
-    model, x1, t = _prepared("intree", cfg, float(G["ratio"][0]), torch.float16)
+    model, x1, t = _prepared(cfg, float(G["ratio"][0]), torch.float16)
     model.set_fused(False)
     with torch.no_grad():
         via_modules = model(x1, t).float()
@@ -166,7 +156,7 @@ def test_fused_step_edit_sweep_vs_reference_golden(tag, tol_max, tol_rms):
     from sige_b200.workloads.ddpm import DDPMConfig
 
     G = golden(tag + "_golden.npz")
-    model, x1, t = _prepared("reference", DDPMConfig(), float(G["ratio"][0]), torch.float32)
+    model, x1, t = _prepared(DDPMConfig(), float(G["ratio"][0]), torch.float32)
     with torch.no_grad():
         out = model(x1, t).float().cpu().numpy()
     assert model.fused_step is not None and model.fused_step.eager_nodes == []
@@ -184,7 +174,7 @@ def test_recompiles_when_masks_or_caches_change():
     from sige_b200.workloads.ddpm import DDPMConfig, synthetic_inputs
 
     cfg = DDPMConfig.small()
-    model, x1, t = _prepared("intree", cfg, 0.05, torch.float16)
+    model, x1, t = _prepared(cfg, 0.05, torch.float16)
     with torch.no_grad():
         a = model(x1, t)
         s1 = model.fused_step
@@ -208,7 +198,7 @@ def test_batch_of_independent_edits_on_gpu():
     from sige_b200.workloads.ddpm import DDPMConfig, synthetic_inputs
 
     cfg = DDPMConfig()
-    model, _, t = _prepared("reference", cfg, 0.012, torch.float32)
+    model, _, t = _prepared(cfg, 0.012, torch.float32)
     edits = []
     for e, (ratio, shift) in enumerate([(0.012, (0, 0)), (0.012, (-70, 45)), (0.03, (60, -80)), (0.006, (-100, -100))]):
         x0, x1, mask, _ = synthetic_inputs(cfg, ratio, seed=0, edit_seed=e)
@@ -240,7 +230,7 @@ def test_set_masks_again_with_the_same_masks_is_free():
     from sige_b200.workloads.ddpm import DDPMConfig, synthetic_inputs
 
     cfg = DDPMConfig.small()
-    model, x1, t = _prepared("intree", cfg, 0.05, torch.float16)
+    model, x1, t = _prepared(cfg, 0.05, torch.float16)
     _, _, mask, _ = synthetic_inputs(cfg, 0.05, seed=0)
     masks = downsample_mask(mask.to(DEV), min_res=8)
     with torch.no_grad():
@@ -267,7 +257,7 @@ def test_multi_step_cached_flow_on_the_fused_path():
     from sige_b200.workloads.ddpm import DDPMConfig, synthetic_inputs
 
     cfg = DDPMConfig.small()
-    model = _model("intree", cfg).to(DEV)
+    model = _model(cfg).to(DEV)
     x0, x1, mask, t = synthetic_inputs(cfg, 0.05, seed=0)
     x0, x1, t = x0.to(DEV), x1.to(DEV), t.to(DEV)
     ids = [0, 1, 2]
@@ -309,7 +299,7 @@ def test_resblock_entry_point_equals_its_two_launches():
     from sige_b200.fused import FusedStep
     from sige_b200.workloads.ddpm import DDPMConfig
 
-    model, x1, t = _prepared("intree", DDPMConfig.small(), 0.05, torch.float16)
+    model, x1, t = _prepared(DDPMConfig.small(), 0.05, torch.float16)
     with torch.no_grad():
         step = FusedStep(model, x1, t, use_graph=False)
     by_name = {f.name: f for f in step.fused}
@@ -342,7 +332,7 @@ def test_next_edit_reuses_the_compiled_step():
     from sige_b200.workloads.ddpm import DDPMConfig, synthetic_inputs
 
     cfg = DDPMConfig()
-    model, x_a, t = _prepared("reference", cfg, 0.012, torch.float32)
+    model, x_a, t = _prepared(cfg, 0.012, torch.float32)
     x0, _, _, _ = synthetic_inputs(cfg, 0.012, seed=0)
     with torch.no_grad():
         out_a = model(x_a, t)
@@ -372,7 +362,7 @@ def test_capacity_headroom_lets_a_larger_mask_in():
     from sige_b200.workloads.ddpm import DDPMConfig, synthetic_inputs
 
     cfg = DDPMConfig.small()
-    model, x_a, t = _prepared("intree", cfg, 0.04, torch.float16)
+    model, x_a, t = _prepared(cfg, 0.04, torch.float16)
     model.set_fused(True, headroom=0.6)
     x0, _, _, _ = synthetic_inputs(cfg, 0.04, seed=0)
     with torch.no_grad():
@@ -397,7 +387,7 @@ def test_next_edit_without_a_host_sync():
     from sige_b200.workloads.ddpm import DDPMConfig, synthetic_inputs
 
     cfg = DDPMConfig.small()
-    model, x_a, t = _prepared("intree", cfg, 0.04, torch.float16)
+    model, x_a, t = _prepared(cfg, 0.04, torch.float16)
     model.set_fused(True, headroom=0.6)
     with torch.no_grad():
         model(x_a, t)
