@@ -108,6 +108,37 @@ def test_conv_in_tiles_matches_dense_inside_the_tiles(dtype):
     assert bool((out[:, :, ~inside] == 7.0).all()) and bool((aux[:, :, ~inside] == 7.0).all())
 
 
+@pytest.mark.parametrize("dtype,tol", [(torch.float16, 1e-3), (torch.bfloat16, 8e-3)])
+def test_conv_in_per_image_tiles_vs_float64(dtype, tol):
+    """sige_conv_in_nhwc_tiles with idx_per_image = 1 (a batch of edits): B = 2, each image with its own list padded with
+    SIGE_TILE_NONE rows; inside each image's own tiles the float64 conv, nothing written anywhere else (not in the other
+    image's tiles either)."""
+    from sige_b200 import ops
+
+    torch.manual_seed(5)
+    B, Cin, Cout, H, W, n, NONE = 2, 3, 128, 40, 36, 6, -30000
+    x = torch.randn(B, Cin, H, W, device=DEV).to(dtype).contiguous(memory_format=torch.channels_last)
+    w = (torch.randn(Cout, Cin, 3, 3, device=DEV) / (Cin * 9) ** 0.5).to(dtype)
+    b = torch.randn(Cout, device=DEV).to(dtype)
+    lists = [[[-1, -1], [3, 7], [35, 31]], [[7, 7], [19, -1], [-1, 27], [11, 15], [23, 3], [35, 11]]]
+    tiles = torch.full((B * n, 2), NONE, dtype=torch.int32)
+    for bi, l in enumerate(lists):
+        tiles[bi * n:bi * n + len(l)] = torch.tensor(l, dtype=torch.int32)
+    out = torch.full((B, Cout, H, W), 7.0, device=DEV, dtype=dtype).contiguous(memory_format=torch.channels_last)
+    ops.conv_in_nhwc(x, w, b, out=out, tiles=tiles.to(DEV), tile_size=6, tiles_per_image=True)
+    want = F.conv2d(x.double().cpu(), w.double().cpu(), b.double().cpu(), 1, 1)
+    inside = torch.zeros(B, 1, H, W, dtype=torch.bool)
+    for bi, l in enumerate(lists):
+        for (y0, x0) in l:
+            inside[bi, :, max(y0, 0):min(y0 + 6, H), max(x0, 0):min(x0 + 6, W)] = True
+    inside = inside.expand(B, Cout, H, W)
+    got = out.double().cpu()
+    err = float((got - want)[inside].abs().max() / want[inside].abs().max())
+    print("conv_in per-image tiles %s: %.3g" % (dtype, err))
+    assert err <= tol
+    assert bool((got[~inside] == 7.0).all()), "written outside the image's own tiles"
+
+
 # Stable Diffusion v1 shapes at a 15 % edit (8 heads x batch 2; head dims 40 / 80 / 160; self-attention against all 4096 / 1024 /
 # 256 / 64 tokens, cross-attention against the 77 text tokens) plus ragged ones (one query, one key, tails that are not a
 # multiple of the 64-row blocks).
